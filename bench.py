@@ -6,7 +6,7 @@ one synthetic stack of independent Conv[512,512,3,3]+BN+ReLU -> Conv[512,512,3,3
 configs[4], the configuration the metric's HBM-roofline half is quoted on; it is the largest single-GPU
 configuration: 4096 layer pairs = 38.65 GB of fp32 weights).  Output: ONE JSON line (see README / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--layers L] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--layers L] [--impl b200|reference] [--dump-outputs DIR]
 
   value      whole-job Conv/BN layer-pairs per second with the stack resident in HBM (device-timed, CUDA events)
   e2e        the same metric through the public API with HOST buffers: pinned host -> device, calibrate, device -> host
@@ -55,6 +55,7 @@ def parse():
                    help="which curve is the line's headline `value` (the other one is reported next to it): weak = --layers "
                         "pairs PER GPU, strong = --layers pairs IN TOTAL split over the GPUs (SURVEY 8(d) config 5)")
     p.add_argument("--no-strong", action="store_true", help="skip the strong-scaling measurement")
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (rank 0)")
     return p.parse_args()
 
 
@@ -192,6 +193,45 @@ def bind_to_gpu_numa_node(local_rank):
         return {"node": node, "cpus": len(cpus), "mempolicy": policy}
     except Exception:
         return None
+
+
+DUMP_CAP = 10 * 2 ** 20 // 4       # floats per dumped array: the six arrays stay under 64 MB together
+
+
+def dump_outputs(out_dir, stack, res):
+    """Write what one calibration step of `stack` computed, as a caller of the path receives it, to out_dir/<name>.npy:
+    the calibrated weights, corrected biases, folded BN vectors (fake_weight / fake_bias) and scale vectors S of every
+    layer, and the sweeps each block took.  An array longer than DUMP_CAP floats is replaced by the same seeded sample of
+    its elements (sorted indices into the concatenation over the layers) on every run, so two builds compare element for
+    element.  The weights of the default stack (38.65 GB) are always sampled."""
+    import numpy as np
+    import torch
+    sess, C, N = stack.sess, stack.C, stack.N
+
+    def sample_index(n):
+        if n <= DUMP_CAP:
+            return torch.arange(n)
+        g = torch.Generator().manual_seed(0)
+        return torch.randint(n, (DUMP_CAP,), generator=g).sort().values
+
+    def gather(offs, n_each):
+        """Elements of the arena windows [off, off + n_each) for off in offs, concatenated (and sampled)."""
+        idx = sample_index(len(offs) * n_each)
+        flat = torch.tensor(offs, dtype=torch.int64)[idx // n_each] + idx % n_each
+        return sess.arena.index_select(0, flat.to(sess.device))
+
+    layers = [sess.layer(li) for li in stack.layers]
+    arrays = {"weights": gather([l["w_off"] for l in layers], N),
+              "bias": gather([l["bias_off"] for l in layers], C),
+              "bn_fake_weight": gather([v["fake_w"] for v in stack.vec], C),
+              "bn_fake_bias": gather([v["fake_b"] for v in stack.vec], C),
+              "scales": gather(list(stack.cle_plan["s_offs"]), C),
+              "sweeps": torch.from_numpy(np.asarray(res.group_sweeps, dtype=np.float64))}
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 * 2 ** 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def one_socket_cores():
@@ -432,6 +472,8 @@ def run_b200(args, rank, world, local_rank):
         res = step(timers)
     barrier()
     clocks = sampler.stop()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, stack, res)
 
     # ---- parity of what was just timed: first and last block of this rank's stack vs the oracle (checker only) ---------
     parity = None

@@ -36,3 +36,28 @@ def test_gpu_arm_without_cuda_fails_loudly():
     r = _run("--steps", "1", "--warmup", "1", "--layers", "8", "--no-e2e", "--no-mbv2", "--no-cpu-baseline", timeout=300)
     assert r.returncode != 0
     assert not [l for l in r.stdout.splitlines() if l.startswith("{") and '"value"' in l]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_exactly_and_steps_are_honoured(tmp_path):
+    """--dump-outputs writes the last timed step's results (float32/float64, <= 64 MB); the same arguments give the same
+    inputs, hence the same outputs, in a second process; --steps sets the timed steps."""
+    import numpy as np
+    flags = ("--layers", "8", "--warmup", "1", "--no-e2e", "--no-mbv2", "--no-cpu-baseline")
+    dumps = []
+    for k, steps in enumerate((2, 5)):
+        out = tmp_path / ("run%d" % k)
+        r = _run("--steps", str(steps), "--dump-outputs", str(out), *flags)
+        assert r.returncode == 0, r.stderr[-3000:]
+        d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert d["steps"] == steps and d["parity_check"]["ok"]
+        dumps.append({p.stem: np.load(p) for p in out.glob("*.npy")})
+    a, b = dumps
+    assert set(a) == {"weights", "bias", "bn_fake_weight", "bn_fake_bias", "scales", "sweeps"}
+    assert sum(x.nbytes for x in a.values()) <= 64 * 2 ** 20
+    assert a["bias"].shape == a["bn_fake_weight"].shape == (8 * 512,) and a["scales"].shape == (4 * 512,)
+    assert a["sweeps"].shape == (4,) and (a["sweeps"] > 0).all()
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64), name
+        assert np.array_equal(a[name], b[name]), name
+        assert np.isfinite(a[name]).all(), name

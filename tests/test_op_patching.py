@@ -5,11 +5,11 @@ The rewrite finds the calling frame with sys._getframe(2) where the reference wa
 the two agree: on a model whose `forward` uses every patched op, the product's patched run (i) calls the functional-op
 observers in the recorded order, each exactly once, with exactly the tensors the ops received, (ii) leaves calls from
 functions not named `forward`, calls on other lines and Tensor.add (one frame deeper, never matched - as in the
-reference) alone, (iii) equals the same forward run under the REFERENCE's own replace_op (live, build container),
-(iv) restores the original attributes.  CPU: oracle-backed executor; -m gpu: the real library on CUDA tensors.
+reference) alone, (iii) equals the same forward run under the REFERENCE's own replace_op (its outputs stored in
+tests/golden/ref_op_patching.npz by tools/make_golden.py), (iv) restores the original attributes.  CPU: oracle-backed
+executor; -m gpu: the real library on CUDA tensors.
 """
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -18,8 +18,6 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 import fakelib
-
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
 
 
 def helper_outside_forward(a, b):
@@ -123,26 +121,25 @@ def test_patched_ops_quantize_exactly_the_recorded_calls_gpu(monkeypatch):
     _check("cuda", monkeypatch, use_fake=False)
 
 
+def reference_run(LT, QuantMeasure):
+    """The forward of _check() under an implementation's replace_op: (outputs, observer order)."""
+    torch.manual_seed(0)
+    model = Net().eval()
+    x = torch.randn(2, 3, 6, 6)
+    out, seen, _ = _run_patched(LT, QuantMeasure, model, x)
+    return out, [i for i, _ in seen]
+
+
 def test_patched_ops_agree_with_the_reference_implementation(monkeypatch):
-    """Same Net object (same source lines), same record and ranges: the product's sys._getframe lookup and the
-    reference's inspect.stack() lookup must quantize the same calls - outputs equal bit for bit (CPU, true division)."""
-    import refenv
-    if not refenv.available():
-        pytest.skip("reference checkout not present")
+    """Same Net (same source lines), same record and ranges: the product's sys._getframe lookup and the reference's
+    inspect.stack() lookup must quantize the same calls - outputs equal bit for bit (CPU, true division) to what the
+    reference's replace_op produced (reference_run)."""
+    gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_op_patching.npz"))
     model, x, ours = _check("cpu", monkeypatch, use_fake=True)
-    saved_path, saved_mods = list(sys.path), dict(sys.modules)
-    try:
-        ref = refenv.install()
-        theirs, seen, _ = _run_patched(ref.layer_transform, ref.quantize.QuantMeasure, model, x)
-    finally:
-        sys.path[:] = saved_path
-        for k in list(sys.modules):     # forget what was imported from the reference tree (not torch's lazy imports)
-            f = getattr(sys.modules[k], "__file__", None) or ""
-            if k not in saved_mods and f.startswith(refenv.REF_ROOT):
-                del sys.modules[k]
-        sys.modules.update(saved_mods)
-    assert [i for i, _ in seen] == list(range(N_OBS))
-    for k, (g, w) in enumerate(zip(ours, theirs)):
+    assert list(gold["observer_order"]) == list(range(N_OBS))
+    assert len(ours) == int(gold["n_outputs"])
+    for k, g in enumerate(ours):
+        w = torch.from_numpy(gold["output_%d" % k])
         assert torch.equal(g, w), ("output", k, (g - w).abs().max())
 
 

@@ -1,6 +1,6 @@
 """Pin the numpy oracle: (1) against fixtures produced by running the reference itself (tests/golden/ref_ops.npz,
-tools/make_golden.py), (2) live against the reference and its checked-in ncnn calibration table when the reference tree
-is present (build container only)."""
+tests/golden/ref_equalization_exact.npz, tools/make_golden.py), (2) live against the reference's checked-in ncnn
+calibration table when the reference tree is present."""
 import os
 import sys
 
@@ -90,7 +90,7 @@ def test_eager_port_agrees_with_numpy_oracle():
 
 
 # ---------------------------------------------------------------------------------------------------------
-# live pins (reference tree present)
+# bit-exact pins (the reference's torch.sqrt injected into the oracle)
 # ---------------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
 def ref():
@@ -110,11 +110,11 @@ CASES = [((32, 16, 3, 3), (24, 32, 3, 3), {}), ((32, 3, 3, 3), (32, 1, 3, 3), {}
          ((96, 16, 1, 1), (96, 1, 3, 3), {}), ((64, 32, 1, 1), (10, 64), {}), ((32, 8, 3, 3), (24, 16, 3, 3), {}),
          ((32, 16, 3, 3), (24, 32, 3, 3), dict(s_range=(0.5, 2.0))), ((32, 16, 3, 3), (24, 32, 3, 3), dict(s_range=(1 / 3.0, 3.0))),
          ((32, 16, 3, 3), (24, 32, 3, 3), dict(eps=1e-3)), ((32, 16, 3, 3), (24, 32, 3, 3), dict(degenerate=True))]
+EQ_NAMES = ("w1", "w2", "b1", "bw", "bb", "S")
 
 
-@pytest.mark.parametrize("s1,s2,opt", CASES)
-@pytest.mark.parametrize("signed", [False, True])
-def test_live_layer_equalization_bit_exact_with_reference_sqrt(ref, s1, s2, opt, signed):
+def equalization_case(s1, s2, opt, signed):
+    """Seeded inputs of one _layer_equalization case: ([w1, w2, b1, bw, bb] as torch tensors, keyword options)."""
     import torch
     torch.manual_seed(hash((s1, s2, signed)) % 1000)
     opt = dict(opt)
@@ -125,11 +125,36 @@ def test_live_layer_equalization_bit_exact_with_reference_sqrt(ref, s1, s2, opt,
         w1[1] = 0; w1[3] = 0.5
         w2.view(s2[0], s2[1], -1)[:, 2] = 0
     b1, bw, bb = torch.randn(s1[0]), torch.rand(s1[0]) + 0.5, torch.randn(s1[0])
-    n = [t.clone().numpy() for t in (w1, w2, b1, bw, bb)]
-    r = ref.dfq._layer_equalization(w1, w2, b1, bw, bb, signed=signed, **opt)
-    S = O.layer_equalization(*n, signed=signed, sqrt_fn=_torch_sqrt, **opt)
-    for got, want in zip(n + [S], [w1, w2, b1, bw, bb, r[3]]):
-        assert np.array_equal(got, want.numpy(), equal_nan=True)
+    return [w1, w2, b1, bw, bb], opt
+
+
+def equalization_digest(a):
+    """sha256 of the float32 bits, every NaN canonical (the pins compare with equal_nan)."""
+    import hashlib
+    a = np.array(a, dtype=np.float32)
+    a[np.isnan(a)] = np.nan
+    return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+@pytest.fixture(scope="module")
+def eq_gold():
+    return np.load(os.path.join(GOLD, "ref_equalization_exact.npz"))
+
+
+@pytest.mark.parametrize("s1,s2,opt", CASES)
+@pytest.mark.parametrize("signed", [False, True])
+def test_live_layer_equalization_bit_exact_with_reference_sqrt(eq_gold, s1, s2, opt, signed):
+    """The reference's _layer_equalization outputs (weights as digests, vectors in full) vs the oracle given the same
+    torch.sqrt: equal bit for bit."""
+    ts, kw = equalization_case(s1, s2, opt, signed)
+    n = [t.numpy() for t in ts]
+    S = O.layer_equalization(*n, signed=signed, sqrt_fn=_torch_sqrt, **kw)
+    key = "c%d_s%d_" % (CASES.index((s1, s2, opt)), signed)
+    for name, got in zip(EQ_NAMES, n + [S]):
+        if name in ("w1", "w2"):
+            assert equalization_digest(got) == str(eq_gold[key + name]), name
+        else:
+            assert np.array_equal(got, eq_gold[key + name], equal_nan=True), name
 
 
 def test_live_golden_ncnn_table(ref):

@@ -15,8 +15,11 @@ build container.  Committed next to its outputs so every fixture can be regenera
   ref_bc_<model>.npz      the reference's dfq.bias_correction ALONE on seed-regenerable inputs (tests/bc_fixture.py):
                           every post-correction bias and fake_bias vector + sha256 of every input tensor
   main_<cls|seg|ssd>.npz  made by tests/main_harness.py --impl reference (the unmodified main scripts end to end)
+  ref_equalization_exact.npz, ref_op_patching.npz, ref_distill.npz
+                          the reference's outputs on the seeded inputs of the bit-exact equalization pins, the
+                          op-patching test and the distilled-data test (pin_fixtures)
 
-usage: python tools/make_golden.py [topology] [mobilenetv2] [resnet18] [deeplab] [ssd] [ops] [bc] [minmax]
+usage: python tools/make_golden.py [topology] [mobilenetv2] [resnet18] [deeplab] [ssd] [ops] [bc] [minmax] [table] [pins]
 """
 import hashlib
 import json
@@ -315,3 +318,38 @@ def ncnn_table_rows():
 
 if __name__ == "__main__" and "table" in sys.argv[1:]:
     ncnn_table_rows()
+
+
+# ---------------------------------------------------------------------------------------------------------
+def pin_fixtures():
+    """What the reference computes on the inputs that three tests build from seeds (the inputs are regenerated by the
+    tests themselves, so only the reference's outputs are stored)."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_distill
+    import test_op_patching
+    import test_oracle_pins as P
+    out = {}
+    for i, (s1, s2, opt) in enumerate(P.CASES):
+        for signed in (False, True):
+            ts, kw = P.equalization_case(s1, s2, opt, signed)
+            r = ref.dfq._layer_equalization(*ts, signed=signed, **kw)
+            key = "c%d_s%d_" % (i, signed)
+            for name, t in zip(P.EQ_NAMES, ts + [r[3]]):
+                out[key + name] = P.equalization_digest(t.numpy()) if name in ("w1", "w2") else t.numpy().copy()
+    np.savez_compressed(os.path.join(GOLD, "ref_equalization_exact.npz"), **out)
+    outs, order = test_op_patching.reference_run(ref.layer_transform, ref.quantize.QuantMeasure)
+    np.savez_compressed(os.path.join(GOLD, "ref_op_patching.npz"), observer_order=np.array(order), n_outputs=np.array(len(outs)),
+                        **{"output_%d" % k: o.numpy() for k, o in enumerate(outs)})
+    import run_main
+    run_main.prepare_environment(use_dropin=False)
+    from ZeroQ.distill_data import getDistilData
+    model = test_distill._tiny()
+    torch.manual_seed(123)
+    batches = getDistilData(model, "imagenet", 2, **test_distill.DISTIL_ARGS)
+    samples, means = test_distill.distil_digest(batches)
+    np.savez_compressed(os.path.join(GOLD, "ref_distill.npz"), n_batches=np.array(len(batches)), **samples, **means)
+    print("pins: %d equalization arrays, %d op-patching outputs, %d distilled batches" % (len(out), len(outs), len(batches)))
+
+
+if __name__ == "__main__" and "pins" in sys.argv[1:]:
+    pin_fixtures()
