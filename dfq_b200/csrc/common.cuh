@@ -131,14 +131,16 @@ __device__ __forceinline__ double warp_sum(double v) {
   return v;
 }
 
-// float atomic min/max through the integer ordering of IEEE bit patterns (works in global and shared).
+// float atomic min/max through the integer ordering of IEEE bit patterns (works in global and shared).  The branch tests the
+// SIGN BIT, not v >= 0: -0.0 (0x80000000) must take the unsigned path of the negatives, where it orders just below +0.0 and
+// above every negative number as fminf/fmaxf do; as a signed int it would be INT_MIN, below -inf.
 __device__ __forceinline__ void atomic_min_f(float* addr, float v) {
-  if (v >= 0.f) atomicMin((int*)addr, __float_as_int(v));
-  else          atomicMax((unsigned int*)addr, __float_as_uint(v));
+  if (__float_as_int(v) >= 0) atomicMin((int*)addr, __float_as_int(v));
+  else                        atomicMax((unsigned int*)addr, __float_as_uint(v));
 }
 __device__ __forceinline__ void atomic_max_f(float* addr, float v) {
-  if (v >= 0.f) atomicMax((int*)addr, __float_as_int(v));
-  else          atomicMin((unsigned int*)addr, __float_as_uint(v));
+  if (__float_as_int(v) >= 0) atomicMax((int*)addr, __float_as_int(v));
+  else                        atomicMin((unsigned int*)addr, __float_as_uint(v));
 }
 
 // ------------------------------------------------------------------------------------------

@@ -96,6 +96,7 @@ CHAINS = [
     [(144, 24, 1, 1), (144, 1, 3, 3), (32, 144, 1, 1)],                                               # inverted residual
     [(64, 32, 3, 3), (64, 64, 3, 3), (48, 64, 3, 3), (10, 48)],                                       # dense chain: re-scanned middles
     [(16, 8, 3, 3), (32, 8, 3, 3), (32, 1, 3, 3), (20, 32, 1, 1)],                                    # grouped (G=2) then depthwise
+    [(1040, 32, 1, 1), (96, 1040, 1, 1), (24, 96, 1, 1)],            # 1040-wide middle: scan and re-scan above 1024 columns
 ]
 
 
@@ -493,7 +494,8 @@ def test_bias_correct_variants_on_mixed_layer_kinds(variant, monkeypatch):
     depthwise (cols = 1, groups = C: one expectation value per row), pointwise with more than 512 columns (expectation
     read from global memory), the 27-float rows of a first conv (tiles the TMA unit cannot move), rows longer than a
     stage (processed in global memory), a 'cat' of two BNs and an 'add' of two BNs, signed and unsigned, the raw-sum
-    (bias absorption) flags - against the oracle, 1e-5 normwise, with and without column-extrema hints."""
+    (bias absorption) flags, and 2049- / 4096-column layers (more expectation values than k_bc_engine caches in shared
+    memory) - against the oracle, 1e-5 normwise."""
     from dfq_b200.engine import Session
     _force_bc_variant(monkeypatch, variant)
     g = torch.Generator().manual_seed(31)
@@ -515,7 +517,14 @@ def test_bias_correct_variants_on_mixed_layer_kinds(variant, monkeypatch):
         (R(12, 32, 3, 3) * 0.1, False, [("A", True, "set")], {}),                          # grouped: 2 groups x 32 columns
         (R(30, 64, 3, 3) * 0.1, False, [("A", False, "set")], dict(raw_sum=True, add=True)),
     ]
-    bns = dict(A=bnA, B=bnB, C=bnC, D=bnD, E=bnE, F=bnF)
+    # wider than the 2048-value expectation cache of k_bc_engine: E[x] read from global memory, the level is not local
+    bnG = (torch.rand(4096, generator=g) + 0.4, R(4096) * 0.5)
+    bnH = (torch.rand(2049, generator=g) + 0.4, R(2049) * 0.5)
+    cases += [
+        (R(10, 4096) * 0.02, False, [("G", True, "set")], {}),                             # linear, 4096 columns
+        (R(8, 2049, 1, 1) * 0.03, True, [("H", False, "set")], {}),                        # 1x1, 2049 columns
+    ]
+    bns = dict(A=bnA, B=bnB, C=bnC, D=bnD, E=bnE, F=bnF, G=bnG, H=bnH)
     sess = Session()
     off = {k: (sess.bind(v[0], False), sess.bind(v[1], False)) for k, v in bns.items()}
     items, biases, lids = [], [], []
